@@ -1,15 +1,17 @@
 #!/usr/bin/env python
 """bench.py -- decode tokens/s of the B200 hot path (BASELINE.json metric) + roofline + CPU baseline.
 
-  python bench.py [--gpus N --steps K --warmup W] [--impl reference]
+  python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 A "step" = one full decode step (all layers: 4 GEMMs + rope/append + paged attention + norms, lm_head, greedy argmax)
 for a batch of synthetic sequences under ONE CUDA graph.  Default workload = the configuration BASELINE.json's metric is
 quoted on: Llama-3-8B INT4-AWQ(g128), batch 32, context 2048, one B200.  N > 1 = the reference's tensor-parallel split
 (strong scaling: the same batch, weights/heads sharded, NCCL all-reduce after the row-parallel GEMMs).
+Weights, KV cache and page tables come from fixed seeds, so --dump-outputs of two builds can be compared array for array.
 """
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -41,7 +43,14 @@ def parse():
     ap.add_argument("--program", type=int, default=int(os.environ.get("B200_PROGRAM", "0")))  # record the step into a decode program (persistent kernel between attention calls)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--comm", default=os.environ.get("B200_COMM", "peer"), choices=["peer", "nccl"])
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's logits and sampled token ids to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl b200: the reference arm does not compute a decode step")
+    return args
 
 
 def peaks():
@@ -67,8 +76,7 @@ def cpu_arm(args, cfg, budget_s=25.0):
     extrapolates to the full step.  kind = "port": the reference snapshot has no CPU backend to compile (SURVEY section 0)."""
     import numpy as np
     from oracle import oracle as orc
-    orc.build()
-    cores = orc.num_threads()
+    cores = orc.num_threads()          # loads the library build() made (compiles it only if it is missing)
     rng = np.random.default_rng(0)
     B, S, T = args.batch, args.ctx, cfg.tokens_per_block
     Hq, Hkv, D, H, I = cfg.head_num, cfg.kv_head_num, cfg.head_dim, cfg.hidden, cfg.inter
@@ -136,8 +144,14 @@ class ClockSampler:
         try:
             self.p = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits", "-lms", "20",
                                        "-i", str(gpu_index)], stdout=self.f, stderr=subprocess.DEVNULL)
+            atexit.register(self._kill)    # a run that fails before stop() must not leave the sampler behind
         except Exception:  # noqa: BLE001
             self.p = None
+
+    def _kill(self):
+        if self.p.poll() is None:
+            self.p.kill()
+            self.p.wait()
 
     def stop(self):
         if self.p is None:
@@ -166,6 +180,43 @@ class ClockSampler:
         sm.sort()
         return dict(sm_mhz=sm[len(sm) // 2] if sm else None, sm_max_mhz=max(mx) if mx else None,
                     reasons=sorted(reasons), samples=len(sm))
+
+
+# ------------------------------------------------------------------------------------------------ outputs
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def step_outputs(model, cfg, tp):
+    """What a caller of the timed step receives from its last run: the logits over the whole vocabulary and the sampled token
+    ids. Under tensor parallelism every rank must call it (the vocab-split logits are gathered)."""
+    import numpy as np
+    import torch
+    import torch.distributed as dist
+    logits = model.logits
+    if tp > 1:
+        parts = [torch.empty_like(logits) for _ in range(tp)]
+        dist.all_gather(parts, logits)
+        logits = torch.cat(parts, dim=1)
+    return {"logits": logits[:, :cfg.vocab].float().cpu().numpy(),
+            "next_ids": model.next_ids.cpu().numpy().astype(np.float64)}
+
+
+def dump_outputs(out_dir, outs):
+    """Writes outs as out_dir/<name>.npy, at most DUMP_LIMIT_BYTES in all. Logits that would not fit keep a fixed, seeded sample
+    of vocabulary columns (the same for every run with the same arguments); their indices go to logits_columns.npy."""
+    import numpy as np
+    outs = dict(outs)
+    logits = outs["logits"]
+    budget = DUMP_LIMIT_BYTES - outs["next_ids"].nbytes - 3 * 1024            # (.npy headers)
+    if logits.nbytes > budget:
+        rows, vocab = logits.shape
+        keep = budget // (rows * logits.itemsize + 8)          # a kept column: its logits + its float64 index
+        cols = np.sort(np.random.default_rng(0).choice(vocab, keep, replace=False))
+        outs["logits"] = np.ascontiguousarray(logits[:, cols])
+        outs["logits_columns"] = cols.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outs.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------ main
@@ -264,6 +315,7 @@ def main():
     en.record()
     barrier()
     ms = st.elapsed_time(en) / args.steps
+    outs = step_outputs(model, cfg, tp) if args.dump_outputs else None
 
     # ---- end to end ("e2e"): host buffers -> H2D -> step -> D2H, every step, through the public call
     for _ in range(3):
@@ -341,6 +393,8 @@ def main():
         if not args.no_cpu_baseline and tp == 1:
             cb = cpu_arm(args, cfg)
             line["cpu_baseline"] = {k: cb[k] for k in ("value", "unit", "cores", "kind", "sample")}
+        if outs is not None:
+            dump_outputs(args.dump_outputs, outs)
         print(json.dumps(line))
     if tp > 1:
         # Teardown: process groups whose collectives were captured in CUDA graphs hang in destroy_process_group

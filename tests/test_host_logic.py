@@ -85,9 +85,12 @@ def test_attn_op_support_gate():
     class I:
         is_prefill = True
     assert attention.B200DecodeAttnOp(C()).support(I()) is False          # decode only
-    C.size_per_head = 64
+    C.size_per_head = 96
     I.is_prefill = False
-    assert attention.B200DecodeAttnOp(C()).support(I()) is False          # head_dim 128 only
+    assert attention.B200DecodeAttnOp(C()).support(I()) is False          # head_dim 64 / 128 / 256 only
+    C.size_per_head = 64
+    on_sm100 = torch.cuda.is_available() and torch.cuda.get_device_capability()[0] == 10
+    assert attention.B200DecodeAttnOp(C()).support(I()) is on_sm100      # a served shape: supported exactly where the kernels run
 
 
 def test_bench_reference_arm_runs_on_cpu_and_prints_the_contract_line():
